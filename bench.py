@@ -18,7 +18,7 @@ Rank 0 prints ONE JSON line:
                        gathered records), i.e. the collective is inside the timed region.
   roofline             per-launch CUDA-event timing of every layer in a SEPARATE profiling pass; `traffic` = measured DRAM
                        bytes per k_conv_tc launch from the committed ncu pass over all launches of one step (profiles/).
-  gpu_eager_baseline   N = 1: the reference's own GPU path on the same box -- its unmodified modules (baseline/_ref, else the
+  gpu_eager_baseline   N = 1: the reference's own GPU path on the same box -- its unmodified modules ($YOLACT_REFERENCE, else the
                        torch restatement in oracle/) .cuda().eval(), cudnn.benchmark=True (eval.py:122-125), TF32 default and
                        bf16 autocast, same batch, CUDA events -- with ours / eager ratios.
   cpu_baseline         N = 1: the reference's CPU path on the host cores, bounded sample.
@@ -28,7 +28,12 @@ Rank 0 prints ONE JSON line:
   mask_stage           after_nms for 100 detections at 480x640 (float32 / uint8 / bit-packed masks), mask IoU and RLE on the packed masks, N = 1.
   training             BASELINE configs[3]: res101 550x550 training step (native engine forward + backward + SGD), bs 2 per GPU, DDP over
                        NCCL at N > 1; at N = 1 beside the same step on torch autograd / cuDNN.
-`--impl reference` times the reference's CPU implementation of the path (the reference itself when staged, else the port).
+`--impl reference` times the reference's CPU implementation of the path (the reference itself when $YOLACT_REFERENCE names a
+checkout of it, else the port).
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float32 / float64): the
+detection records det_count, det_cls, det_anchor, det_score, det_box, det_coef (rank 0; all ranks' records at N > 1), and the
+network outputs cls, box, coef, proto (rank 0's shard; arrays above DUMP_SAMPLE elements as a fixed seeded sample of flat
+positions).  Inputs and weights are seeded, so two builds run with the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -119,8 +124,8 @@ class ClockSampler:
 # reference arm / cpu_baseline: the reference's CPU path (eval forward + nms() per image), fp32, all host threads
 # ----------------------------------------------------------------------------------------------------
 def cpu_reference_sample(arch, img_size, n_img, reps, threads):
-    """Returns (img_per_s, seconds, fast_nms_us_per_img, kind).  kind = 'reference' when the unmodified reference is staged
-    (baseline/_ref: its Yolact.forward + utils/output_utils.nms, FPN run-time patch for sizes % 32 != 0), else 'port' (oracle/)."""
+    """Returns (img_per_s, seconds, fast_nms_us_per_img, kind).  kind = 'reference' when the unmodified reference is available
+    ($YOLACT_REFERENCE: its Yolact.forward + utils/output_utils.nms, FPN run-time patch for sizes % 32 != 0), else 'port' (oracle/)."""
     import torch
     from oracle import synth, forward_torch as ft, postprocess_np as pp, ref_loader
     torch.set_num_threads(threads)
@@ -168,7 +173,7 @@ def run_reference(args):
         v, dt, nu, kind = cpu_reference_sample(ARCH, IMG, n_img, 1, cores)
         vals.append(v); t_all += dt; nms_us = nu
     value = float(np.mean(vals))
-    what = ('the UNMODIFIED reference (baseline/_ref: Yolact.forward + utils/output_utils.nms' + (', FPN interpolate-to-size run-time patch for 550' if IMG % 32 else '') + ')'
+    what = ('the UNMODIFIED reference ($YOLACT_REFERENCE: Yolact.forward + utils/output_utils.nms' + (', FPN interpolate-to-size run-time patch for 550' if IMG % 32 else '') + ')'
             if kind == 'reference' else 'CPU port of the reference path (oracle/)')
     line = {'impl': 'reference', 'metric': 'img/s', 'value': value, 'unit': 'img/s', 'n_gpus': args.gpus, 'steps': steps,
             'warmup': args.warmup, 'ms_per_step': 1e3 * t_all / steps, 'higher_is_better': True, 'scaling': 'weak',
@@ -194,6 +199,28 @@ def cuda_time(fn, reps):
     return a.elapsed_time(b) / reps                                  # ms per call
 
 
+DUMP_SAMPLE = 1 << 20     # elements kept of each network output by --dump-outputs: 4 x 4 MB, beside ~1 MB of detection records
+
+
+def dump_outputs(dirname, outs, det):
+    """--dump-outputs: the network outputs (cls, box, coef, proto) and the detection records (det_*) of one step as .npy files.
+    An output above DUMP_SAMPLE elements is written as the values at the sorted flat positions np.unique of DUMP_SAMPLE draws
+    from default_rng(0), the same positions in every run of the same shape."""
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {}
+    for name, t in zip(('cls', 'box', 'coef', 'proto'), outs):
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), DUMP_SAMPLE))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        arrays[name] = t.float().cpu().numpy()
+    for k in ('count', 'cls', 'anchor', 'score', 'box', 'coef'):
+        a = det[k].cpu().numpy()
+        arrays['det_' + k] = a.astype(np.float64 if a.dtype.kind in 'iu' else np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 def gpu_eager_baseline(arch, img_size, batch, dev, our_img_s, steps=5):
     """The reference's own GPU path, on this box: eager PyTorch / cuDNN, as eval.py:122-125 runs it."""
     import torch
@@ -209,7 +236,7 @@ def gpu_eager_baseline(arch, img_size, batch, dev, our_img_s, steps=5):
             net, _ = ref_loader.build_net(arch, img_size, sd)
             net = net.to(dev)
             fwd = lambda: net(x)
-            out['impl'] = 'unmodified reference modules (baseline/_ref)' + (' + FPN interpolate-to-size run-time patch' if img_size % 32 else '')
+            out['impl'] = 'unmodified reference modules ($YOLACT_REFERENCE)' + (' + FPN interpolate-to-size run-time patch' if img_size % 32 else '')
         else:
             sdd = {k: v.to(dev) for k, v in sd.items()}
             fwd = lambda: ft.forward(x, sdd, arch)
@@ -486,6 +513,8 @@ def run_ours(args):
     state = drain()
     outs, det = state['outs'], state['det']
     gathered = state['pending'].result() if world > 1 else det
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs, gathered)
     value = world * per_gpu[main_mode] * K / (ms / 1e3)
 
     # ---- the other scaling mode in the same run (N > 1) -------------------------------------------------
@@ -753,7 +782,10 @@ if __name__ == '__main__':
     ap.add_argument('--arch', default=ARCH, choices=['res101', 'res50', 'swin_tiny'], help='default: the BASELINE metric config')
     ap.add_argument('--img', type=int, default=IMG)
     ap.add_argument('--batch', type=int, default=BATCH, help='images per GPU (weak) / global batch (strong)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write what the last timed step computed to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     ARCH, IMG, BATCH = args.arch, args.img, args.batch
     if args.eager_train_leg:
         import torch

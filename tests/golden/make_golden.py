@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Golden-vector generator (TEST INFRASTRUCTURE).  Runs ONLY in the build container, where the
-read-only reference checkout exists at /root/reference; the fixtures it writes next to this
-file are committed and are what travels to the GPU box.
+"""Golden-vector generator (TEST INFRASTRUCTURE).  Needs a checkout of the reference, named by
+$YOLACT_REFERENCE; the fixtures it writes next to this file are committed, so the tests never
+need the reference itself.
 
-  python tests/golden/make_golden.py            # regenerate every fixture
+  YOLACT_REFERENCE=<checkout> python tests/golden/make_golden.py            # regenerate every fixture
 
 It imports the UNMODIFIED reference modules (modules.yolact.Yolact, utils.output_utils.nms /
 after_nms, utils.box_utils.make_anchors) and, for the traditional-NMS path, a copy of
@@ -21,7 +21,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = os.environ.get('YOLACT_REFERENCE', '/root/reference')
+REF = os.environ['YOLACT_REFERENCE']
 REFBUILD = os.path.join(ROOT, 'oracle', '_ref')
 sys.path.insert(0, ROOT)
 
@@ -243,11 +243,13 @@ def patch_fpn(ryolact):
 
 
 def gen_forward(rcfg, ryolact):
+    # strides keep the fixture small: about 40 anchor rows (every aspect ratio: sub is not a multiple of 3) and a 6 x 6
+    # grid of proto pixels per image
     out = {}
-    cases = [('res50', 64, 2, 1, False), ('res101', 64, 1, 1, False), ('res50', 128, 2, 4, False),
-             ('res50', 400, 1, 16, True), ('res101', 544, 1, 32, False), ('res101', 550, 1, 32, True),
-             ('swin_tiny', 96, 2, 1, False), ('swin_tiny', 224, 1, 8, False), ('swin_tiny', 550, 1, 32, True)]
-    for arch, S, B, sub, need_patch in cases:
+    cases = [('res50', 64, 2, 7, 3, False), ('res101', 64, 1, 7, 3, False), ('res50', 128, 2, 25, 5, False),
+             ('res50', 400, 1, 250, 17, True), ('res101', 544, 1, 463, 23, False), ('res101', 550, 1, 481, 23, True),
+             ('swin_tiny', 96, 2, 14, 4, False), ('swin_tiny', 224, 1, 79, 9, False), ('swin_tiny', 550, 1, 481, 23, True)]
+    for arch, S, B, sub, psub, need_patch in cases:
         cfg = ref_cfg(rcfg, arch + '_coco', S)
         sd = ft.synth_state_dict(arch, seed=0)
         net = ryolact.Yolact(cfg)
@@ -265,10 +267,11 @@ def gen_forward(rcfg, ryolact):
         key = f'{arch}_S{S}_B{B}'
         cls, box, coef, proto = [t.numpy() for t in ref]
         out[key + '/sub'] = np.int64(sub)
+        out[key + '/psub'] = np.int64(psub)
         out[key + '/cls'] = cls[:, ::sub]
         out[key + '/box'] = box[:, ::sub]
         out[key + '/coef'] = coef[:, ::sub]
-        out[key + '/proto'] = proto[:, ::sub, ::sub]
+        out[key + '/proto'] = proto[:, ::psub, ::psub]
         out[key + '/shapes'] = np.asarray([cls.shape[1], proto.shape[1]], dtype=np.int64)
         print(f'  forward {key}: A={cls.shape[1]} P={proto.shape[1]} oracle-vs-reference max err {max(errs):.2e}')
     np.savez_compressed(os.path.join(HERE, 'forward.npz'), **out)

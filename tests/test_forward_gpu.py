@@ -60,11 +60,11 @@ def test_forward_fp32_small_vs_oracle_golden_and_taps(cuda, arch, S, B):
         assert np.abs(t - r).max() < 1e-3 * max(1.0, np.abs(r).max()), (tap, rel_err(t, r))
     g = load_golden('forward.npz')
     key = f'{arch}_S{S}_B{B}'
-    sub = int(g[key + '/sub'])
+    sub, psub = int(g[key + '/sub']), int(g[key + '/psub'])
     assert np.abs(mine[0][:, ::sub] - g[key + '/cls']).max() < TOL['fp32']
     assert np.abs(mine[1][:, ::sub] - g[key + '/box']).max() < TOL['fp32']
     assert np.abs(mine[2][:, ::sub] - g[key + '/coef']).max() < TOL['fp32']
-    assert np.abs(mine[3][:, ::sub, ::sub] - g[key + '/proto']).max() < TOL['fp32']
+    assert np.abs(mine[3][:, ::psub, ::psub] - g[key + '/proto']).max() < TOL['fp32']
     assert np.array_equal(net.engine(B).anchors(), pp.make_anchors(S))
 
 
@@ -76,9 +76,9 @@ def test_forward_fp32_full_size_vs_golden(cuda, arch, S):
     mine = run(net, img, cuda)
     g = load_golden('forward.npz')
     key = f'{arch}_S{S}_B1'
-    sub = int(g[key + '/sub'])
+    sub, psub = int(g[key + '/sub']), int(g[key + '/psub'])
     assert mine[0].shape[1] == int(g[key + '/shapes'][0]) and mine[3].shape[1] == int(g[key + '/shapes'][1])
-    for m, name in ((mine[0][:, ::sub], 'cls'), (mine[1][:, ::sub], 'box'), (mine[2][:, ::sub], 'coef'), (mine[3][:, ::sub, ::sub], 'proto')):
+    for m, name in ((mine[0][:, ::sub], 'cls'), (mine[1][:, ::sub], 'box'), (mine[2][:, ::sub], 'coef'), (mine[3][:, ::psub, ::psub], 'proto')):
         assert np.abs(m - g[f'{key}/{name}']).max() < TOL['fp32'], (name, rel_err(m, g[f'{key}/{name}']))
 
 

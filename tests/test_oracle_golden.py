@@ -70,12 +70,12 @@ def test_forward_golden_small(key):
     g = load_golden('forward.npz')
     arch, S, B = key.split('_')
     S, B = int(S[1:]), int(B[1:])
-    sub = int(g[key + '/sub'])
+    sub, psub = int(g[key + '/sub']), int(g[key + '/psub'])
     sd = ft.synth_state_dict(arch, seed=0)
     img = torch.from_numpy(synth.image_batch(11, B, S))
     cls, box, coef, proto = [t.numpy() for t in ft.forward(img, sd, arch)]
     assert cls.shape[1] == int(g[key + '/shapes'][0]) and proto.shape[1] == int(g[key + '/shapes'][1])
-    for mine, name in ((cls[:, ::sub], 'cls'), (box[:, ::sub], 'box'), (coef[:, ::sub], 'coef'), (proto[:, ::sub, ::sub], 'proto')):
+    for mine, name in ((cls[:, ::sub], 'cls'), (box[:, ::sub], 'box'), (coef[:, ::sub], 'coef'), (proto[:, ::psub, ::psub], 'proto')):
         assert np.allclose(mine, g[f'{key}/{name}'], rtol=0, atol=2e-6), name
 
 
